@@ -5,6 +5,7 @@ oracle timed beside it.
 
   python bench.py [--gpus N] [--steps K] [--warmup W]              # torchrun launches one rank per GPU for N>1
   python bench.py --impl reference [--gpus N] [--steps K] ...      # the CPU arm (oracle port; pybullet is absent)
+  python bench.py ... --dump-outputs DIR                           # also save what the last timed step returned, DIR/<name>.npy
 
 A "step" is one env.step() over the whole env batch of a rank (= 13 fused physics substeps + ETG + obs/reward pack in
 ONE kernel launch).  Weak scaling: every rank owns its own 4096 envs, no data-path collective.
@@ -28,6 +29,7 @@ WORKLOAD = "BASELINE configs[1]: 4096 parallel A1 envs per GPU, flat terrain, fi
 ALG_BYTES_IN = 21 * 16 + 15 * 16 + 16 * 16 + 48 + 4 + 2 * 3 * 4 * 16      # state, params, ETG, action, counter, history reads
 ALG_BYTES_OUT = 21 * 16 + 2 * 3 * 4 * 16 + 49 * 4 + 4 + 1 + 56 * 4 + 4      # state, history writes, obs, reward, done, info, counter
 ALG_BYTES_PER_ENV_STEP = ALG_BYTES_IN + ALG_BYTES_OUT
+DUMP_BYTES = 60 * 10 ** 6                    # --dump-outputs payload cap: the files, headers included, stay under 64 MB
 
 
 def etg_weights():
@@ -105,6 +107,18 @@ def cpu_oracle_rate(n_envs, steps, threads, w, b, seed=1234):
     batch.rollout(acts, auto_reset=True, nthreads=threads)
     dt = time.perf_counter() - t0
     return n_envs * steps / dt, dt
+
+
+def dump_outputs(out_dir, outputs, suffix=""):
+    """Saves the arrays one env.step() returned as out_dir/<name><suffix>.npy in float32, so that two builds can be compared output for
+    output.  Above DUMP_BYTES in all, a fixed seeded sample of env rows (the same rows for the same env count) stands for the batch."""
+    n = next(iter(outputs.values())).shape[0]
+    row_bytes = 4 * sum(t[0].numel() for t in outputs.values())
+    keep = min(n, DUMP_BYTES // row_bytes)
+    rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False)) if keep < n else slice(None)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(os.path.join(out_dir, name + suffix + ".npy"), t.float().cpu().numpy()[rows])
 
 
 def run_reference(args):
@@ -306,7 +320,12 @@ def main():
     ap.add_argument("--envs", type=int, default=ENVS_PER_GPU)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the BASELINE configs[2..4] / strong-scaling block")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write obs / reward / done / info of the last timed step to DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs saves the GPU path's outputs; the reference arm has none")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -354,6 +373,8 @@ def main():
     total_ms = float(t[0])
     value = world * n * K / (total_ms * 1e-3)
     done_frac = float(env.done.float().mean())
+    if args.dump_outputs:                                    # before the host-API leg below steps the same env again
+        dump_outputs(args.dump_outputs, {"obs": env.obs, "reward": env.reward, "done": env.done, "info": env.info}, "" if world == 1 else "_rank%d" % rank)
 
     # end to end through the host-facing API: pinned H2D of the actions + step + D2H of obs/reward/done every step
     host_acts = np.random.default_rng(1234 + rank).uniform(-0.3, 0.3, (16, n, 12)).astype(np.float32)

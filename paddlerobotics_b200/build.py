@@ -5,7 +5,7 @@ import subprocess
 CSRC = os.path.join(os.path.dirname(os.path.abspath(__file__)), "csrc")
 LIB = os.path.join(CSRC, "libb2q.so")
 SOURCES = ["b2q_api.cu", "b2q_mlp.cu", "b2q_es.cu", "b2q_sac.cu", "b2q_rpm.cu"]
-HEADERS = ["b2q_sim.cuh", "b2q_math.cuh", "b2q_host_common.h", "b2q_model_host.h", "b2q_tc.cuh", "../../include/b2q.h", "../../include/b2q_mlp.h", "../../include/b2q_es.h", "../../include/b2q_sac.h", "../../include/b2q_rpm.h", "b2q_mlp_internal.h"]
+HEADERS = ["b2q_sim.cuh", "b2q_math.cuh", "b2q_host_common.h", "b2q_model_host.h", "b2q_tc.cuh", "b2q_philox.cuh", "../../include/b2q.h", "../../include/b2q_mlp.h", "../../include/b2q_es.h", "../../include/b2q_sac.h", "../../include/b2q_rpm.h", "b2q_mlp_internal.h"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17", "-Xcompiler", "-fPIC", "-shared"]
 
 

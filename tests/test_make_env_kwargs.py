@@ -26,9 +26,6 @@ def test_other_env_names_raise():
 
 
 def test_unknown_keyword_is_a_type_error_not_ignored():
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("needs the CPU-only box: on a GPU the engine config check is covered by the gpu tests")
     with pytest.raises((TypeError, RuntimeError)):
         _mk(task="ground", no_such_option=1)
 
